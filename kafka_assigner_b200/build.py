@@ -12,11 +12,15 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
               "-shared", "-Xcompiler", "-fPIC"]
 
 
-def _nvcc():
-    for cand in (shutil.which("nvcc"), "/usr/local/cuda/bin/nvcc"):
+def cuda_tool(name):
+    """Path of a CUDA toolkit program (nvcc, cuobjdump): PATH first, then $CUDA_HOME/bin, then /usr/local/cuda/bin,
+    so that an account whose PATH lacks the toolkit still finds it."""
+    homes = [os.environ.get("CUDA_HOME"), os.environ.get("CUDA_PATH"), "/usr/local/cuda"]
+    for cand in [shutil.which(name)] + [os.path.join(h, "bin", name) for h in homes if h]:
         if cand and os.path.exists(cand):
             return cand
-    raise RuntimeError("nvcc not found: libkassign.so cannot be built (there is no CPU fallback)")
+    raise RuntimeError("%s not found: put the CUDA toolkit's bin/ on PATH or set CUDA_HOME "
+                       "(libkassign.so has no CPU fallback)" % name)
 
 
 HOST_DIR = os.path.join(_HERE, "host")
@@ -51,7 +55,7 @@ def build(force=False, verbose=False):
     """Compile every CUDA source into csrc/libkassign.so. Cross-compiles without a GPU."""
     if not force and not needs_build():
         return LIB
-    cmd = [_nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + SOURCES
+    cmd = [cuda_tool("nvcc")] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + SOURCES
     subprocess.check_call(cmd, cwd=CSRC)
     return LIB
 

@@ -5,6 +5,7 @@ Importers allowed: tests/, __graft_entry__.smoke(), bench.py (cpu_baseline / --i
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -22,10 +23,20 @@ class OracleStatus(ctypes.Structure):
                 ("a", ctypes.c_int32), ("b", ctypes.c_int32), ("message", ctypes.c_char * 256)]
 
 
+def _compile(src, lib):
+    """g++ `src` into `lib`; when oracle/ is read-only (a shared checkout), into a fresh temporary directory instead.
+    Returns the path written."""
+    if not os.access(os.path.dirname(lib), os.W_OK):
+        lib = os.path.join(tempfile.mkdtemp(prefix="kassign-oracle-"), os.path.basename(lib))
+    subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", lib, src])
+    return lib
+
+
 def build(force=False):
     """g++ the restatements into oracle/liboracle.so + libfastoracle.so (gcc only; no reference sources are copied)."""
+    global _LIB
     if force or not os.path.exists(_LIB) or os.path.getmtime(_LIB) < os.path.getmtime(_SRC):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", _LIB, _SRC])
+        _LIB = _compile(_SRC, _LIB)
     fast_lib()
     return _LIB
 
@@ -45,10 +56,10 @@ _flib = None
 
 def fast_lib():
     """The optimised flat-array CPU solver (fast_oracle.cpp) — BASELINE.md 'B1' and a third restatement."""
-    global _flib
+    global _flib, _FLIB
     if _flib is None:
         if not os.path.exists(_FLIB) or os.path.getmtime(_FLIB) < os.path.getmtime(_FSRC):
-            subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", _FLIB, _FSRC])
+            _FLIB = _compile(_FSRC, _FLIB)
         L = ctypes.CDLL(_FLIB)
         L.fast_ctx_create.restype = ctypes.c_void_p
         L.fast_ctx_destroy.argtypes = [ctypes.c_void_p]

@@ -30,7 +30,8 @@ def test_library_exports_every_declared_symbol(native_lib):
 
 def test_library_is_sm100a_cuda_not_a_cpu_build():
     import subprocess
-    out = subprocess.run(["cuobjdump", "--list-elf", kab.lib_path()], capture_output=True, text=True).stdout
+    out = subprocess.run([kab.build_mod.cuda_tool("cuobjdump"), "--list-elf", kab.lib_path()], capture_output=True,
+                         text=True).stdout
     assert "sm_100a" in out
 
 

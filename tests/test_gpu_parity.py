@@ -484,52 +484,54 @@ def test_degenerate_shapes(native_lib, oracle):
         kab.KafkaTopicAssigner().generate_assignment("big", {0: list(range(1, 10))}, set(range(1, 12)), {}, -1)  # 9 replicas > 8 slots
 
 
-def test_rack_pointer_spread_variant_is_exact(native_lib, oracle):
+def test_rack_pointer_spread_variant_is_exact(native_lib, oracle, tmp_path):
     """The opt-in per-rack-pointer spread (KA_SPREAD_RACKPTR=1) must give the same bytes as the default window scan."""
     import subprocess
     import sys
-    code = ("import numpy as np, kafka_assigner_b200 as kab\n"
+    code = ("import os, sys, numpy as np, kafka_assigner_b200 as kab\n"
             "for key, kind in (('c1','random'), ('c2','mixed')):\n"
             "    cl = kab.synth.make_config(key, kind)\n"
             "    out, _, st = kab.Solver(0).solve_cluster(cl)\n"
-            "    np.save('/tmp/_rp_%s.npy' % key, out)\n")
+            "    np.save(os.path.join(sys.argv[1], '_rp_%s.npy' % key), out)\n")
     env = dict(os.environ, KA_SPREAD_RACKPTR="1", PYTHONPATH=util.os.path.dirname(util.HERE))
-    subprocess.run([sys.executable, "-c", code], check=True, env=env, timeout=300)
+    subprocess.run([sys.executable, "-c", code, str(tmp_path)], check=True, env=env, timeout=300)
     for key, kind in (("c1", "random"), ("c2", "mixed")):
         cl = kab.synth.make_config(key, kind)
         exp, _, _ = util.oracle_dense(oracle, cl)
-        assert np.array_equal(np.load("/tmp/_rp_%s.npy" % key).reshape(-1, 3), exp)
+        assert np.array_equal(np.load(tmp_path / ("_rp_%s.npy" % key)).reshape(-1, 3), exp)
 
 
-def test_pipelined_super_chunks_are_exact(native_lib, oracle):
+def test_pipelined_super_chunks_are_exact(native_lib, oracle, tmp_path):
     """KA_PIPELINE_STAGES=3 forces the two-stream super-chunk pipeline on small problems: same bytes, same counters,
     and a failure in a later chunk is reported with its GLOBAL topic index."""
     import subprocess
     import sys
-    code = ("import numpy as np, kafka_assigner_b200 as kab\n"
+    code = ("import os, sys, numpy as np, kafka_assigner_b200 as kab\n"
+            "d = sys.argv[1]\n"
             "for key, kind in (('c1','mixed'), ('c2','mixed'), ('c2','random')):\n"
             "    cl = kab.synth.make_config(key, kind)\n"
             "    s = kab.Solver(0)\n"
             "    out, out_len, st = s.solve_cluster(cl)\n"
-            "    np.save('/tmp/_pl_%s_%s.npy' % (key, kind), out); np.save('/tmp/_plc_%s_%s.npy' % (key, kind), s.counters())\n"
+            "    np.save(os.path.join(d, '_pl_%s_%s.npy' % (key, kind)), out)\n"
+            "    np.save(os.path.join(d, '_plc_%s_%s.npy' % (key, kind)), s.counters())\n"
             "bad = kab.synth.make_cluster(T=30, P=48, RF=3, N=60, R=6, seed=21, kind='mixed', rack_aware=False, remove_frac=0.2, n_old=60)\n"
             "_, _, st = kab.Solver(0).solve_cluster(bad, check=False)\n"
-            "np.save('/tmp/_pl_bad.npy', np.array([st.code, st.topic_index, st.partition]))\n")
+            "np.save(os.path.join(d, '_pl_bad.npy'), np.array([st.code, st.topic_index, st.partition]))\n")
     env = dict(os.environ, KA_PIPELINE_STAGES="3", PYTHONPATH=util.os.path.dirname(util.HERE))
-    subprocess.run([sys.executable, "-c", code], check=True, env=env, timeout=300)
+    subprocess.run([sys.executable, "-c", code, str(tmp_path)], check=True, env=env, timeout=300)
     for key, kind in (("c1", "mixed"), ("c2", "mixed"), ("c2", "random")):
         cl = kab.synth.make_config(key, kind)
         octx = oracle.OracleContext()
         exp, _, _ = util.oracle_dense(oracle, cl, octx)
-        assert np.array_equal(np.load("/tmp/_pl_%s_%s.npy" % (key, kind)).reshape(-1, 3), exp), (key, kind)
-        ctr = np.load("/tmp/_plc_%s_%s.npy" % (key, kind))
+        assert np.array_equal(np.load(tmp_path / ("_pl_%s_%s.npy" % (key, kind))).reshape(-1, 3), exp), (key, kind)
+        ctr = np.load(tmp_path / ("_plc_%s_%s.npy" % (key, kind)))
         for i in range(0, cl.N, 7):
             for slot in range(3):
                 assert ctr[i, slot] == octx.counter(int(cl.broker_id[i]), slot)
     bad = kab.synth.make_cluster(T=30, P=48, RF=3, N=60, R=6, seed=21, kind="mixed", rack_aware=False, remove_frac=0.2, n_old=60)
     _, _, est = util.oracle_dense(oracle, bad)
     assert est.code == 4 and est.topic_index >= 10      # fails in the 2nd or 3rd chunk of 3
-    assert np.load("/tmp/_pl_bad.npy").tolist() == [est.code, est.topic_index, est.partition]
+    assert np.load(tmp_path / "_pl_bad.npy").tolist() == [est.code, est.topic_index, est.partition]
 
 
 def test_broker_tables_beyond_shared_memory(native_lib, oracle):
