@@ -118,6 +118,15 @@ int32_t ka_solve_dense_json(ka_ctx* ctx, int32_t T, const int32_t* topic_hash, i
                             const int32_t* cur_broker, int32_t desired_rf, const char* names, const int64_t* name_off,
                             char* json, int64_t json_cap, int64_t* json_bytes, ka_status* st);
 
+/* Same as ka_solve_dense_json, but the text lists only the rows the solve changes (movement class != UNCHANGED, see
+ * ka_plan_last below), in the same order and format: {"partitions":[],"version":1} when nothing changes.
+ * kafka-reassign-partitions accepts any subset of the partitions, so this is the reassignment to apply. Every finished
+ * block of rows is classified and compacted on the device; only the changed rows' text crosses PCIe. The json_cap rules
+ * and KA_ERR_LIMIT are those of ka_solve_dense_json. */
+int32_t ka_solve_dense_json_changed(ka_ctx* ctx, int32_t T, const int32_t* topic_hash, int32_t P, int32_t RF,
+                                    const int32_t* cur_broker, int32_t desired_rf, const char* names, const int64_t* name_off,
+                                    char* json, int64_t json_cap, int64_t* json_bytes, ka_status* st);
+
 /* Dense form on DEVICE buffers (d_* are device pointers on the ctx's device; d_out_len may be NULL),
  * enqueued on `stream` (a cudaStream_t, NULL = the legacy default stream) — inputs already resident in
  * HBM, outputs left in HBM. If st != NULL the call synchronises the stream and fills *st; with
@@ -159,6 +168,38 @@ int32_t ka_ctx_set_topic_base(ka_ctx* ctx, int32_t topic_base);
 
 /* Synchronise the last asynchronous solve and return its status. */
 int32_t ka_last_status(ka_ctx* ctx, ka_status* st);
+
+/* ---- movement plan ------------------------------------------------------------------------------
+ * What applying the last solve's assignment moves. Row g has current list C (leader first; dense cur[g*RF ..] or ragged
+ * cur_broker[rep_off[g] ..]) and new list O (out_len[g] long, or the target RF when the solve had no out_len). Its class:
+ *   0 UNCHANGED  O == C as sequences
+ *   1 REORDERED  same broker set and length, other order: only the preferred leader / fallback order changes, no data copied
+ *   2 MOVED      the broker sets or the lengths differ (an empty C is MOVED)
+ * added = |O \ C|, dropped = |C \ O| (as sets; a broker repeated in C counts once); leader changed = O[0] != C[0] (with an
+ * empty C, O[0] is a leader gain). */
+typedef struct ka_plan_totals {
+    int64_t rows, rows_reordered, rows_moved, replicas_added, replicas_dropped, leaders_changed;
+} ka_plan_totals;
+
+/* Report-id list of ka_plan_last's per-broker columns: ids[M] strictly ascending, M <= 65534. M = 0 (the default): the live
+ * broker table of the moment ka_plan_last runs. Brokers being decommissioned are not live: list them here to see them one
+ * by one. */
+int32_t ka_ctx_set_report_brokers(ka_ctx* ctx, int32_t M, const int32_t* ids);
+
+/* Movement plan of the ctx's last successful solve (ka_solve, ka_solve_dense, ka_solve_dense_json[_changed],
+ * ka_solve_dense_device), computed on the device from the rows still resident: no second upload. After
+ * ka_solve_dense_device the caller's d_cur_broker / d_out_broker / d_out_len must still hold what that solve read and wrote.
+ * Synchronises the last solve first, like ka_last_status. KA_ERR_BAD_ARG before any solve, after a failed solve and after the
+ * split stage / order / emit solve.
+ *   row_class[Q]          class of every row (NULL: not wanted)
+ *   broker_stats[(M+1)*8] per report bucket (row i < M: ids[i]; row M: every other id), uint32 columns
+ *                         replicas_before, replicas_after, replicas_in, replicas_out,
+ *                         leaders_before, leaders_after, leaders_in, leaders_out   (NULL: not wanted)
+ *   totals                (NULL: not wanted)
+ * Per bucket after = before + in - out (replicas and leaders); sum(replicas_in) = replicas_added, sum(replicas_out) =
+ * replicas_dropped, sum(leaders_in) = leaders_changed, sum(leaders_out) = leaders_changed - (rows with an empty C that got a
+ * leader). */
+int32_t ka_plan_last(ka_ctx* ctx, uint8_t* row_class, uint32_t* broker_stats, ka_plan_totals* totals);
 
 /* ---- counters (Context.counter) -----------------------------------------------------------------
  * counter[i*slots + r] = Context.counter[broker_id[i]][r] for the CURRENT broker table (KAS:289-301:

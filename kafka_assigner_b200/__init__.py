@@ -10,6 +10,7 @@ from . import synth  # noqa: F401
 from ._native import KaStatus, load as load_native, lib_path  # noqa: F401
 from .assigner import (ArrayIndexOutOfBoundsException, IllegalStateException, KafkaTopicAssigner,  # noqa: F401
                        KassignError, Solver, java_string_hash, raise_for_status)
+from .assigner import PLAN_COLUMNS, ROW_MOVED, ROW_REORDERED, ROW_UNCHANGED  # noqa: F401
 
 __all__ = ["KafkaTopicAssigner", "Solver", "IllegalStateException", "ArrayIndexOutOfBoundsException",
            "KassignError", "java_string_hash", "synth", "load_native", "lib_path", "KaStatus", "raise_for_status"]

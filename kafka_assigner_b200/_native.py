@@ -11,6 +11,11 @@ class KaStatus(ctypes.Structure):
                 ("a", ctypes.c_int32), ("b", ctypes.c_int32)]
 
 
+class KaPlanTotals(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int64) for n in ("rows", "rows_reordered", "rows_moved", "replicas_added", "replicas_dropped",
+                                              "leaders_changed")]
+
+
 KA_OK = 0
 KA_ERR_RF_MISMATCH, KA_ERR_RF_NOT_POSITIVE, KA_ERR_RF_GT_BROKERS, KA_ERR_UNASSIGNABLE, KA_ERR_HASH_INDEX = 1, 2, 3, 4, 5
 KA_ERR_BAD_ARG, KA_ERR_CUDA, KA_ERR_NO_DEVICE, KA_ERR_LIMIT = -1, -2, -3, -4
@@ -27,6 +32,7 @@ SYMBOLS = {
     "ka_solve": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]),
     "ka_solve_dense": (_i32, [_vp, _i32, _vp, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _vp]),
     "ka_solve_dense_json": (_i32, [_vp, _i32, _vp, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp]),
+    "ka_solve_dense_json_changed": (_i32, [_vp, _i32, _vp, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp]),
     "ka_solve_dense_device": (_i32, [_vp, _i32, _vp, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
     "ka_stage_dense_device": (_i32, [_vp, _i32, _vp, _i32, _i32, _vp, _i32, _i32, _vp]),
     "ka_order_device": (_i32, [_vp, _vp, _vp, _vp, _vp]),
@@ -37,6 +43,8 @@ SYMBOLS = {
     "ka_ctx_export_counter_slot_device": (_i32, [_vp, _i32, _vp, _vp]),
     "ka_ctx_import_counter_slot_device": (_i32, [_vp, _i32, _vp, _vp]),
     "ka_last_status": (_i32, [_vp, _vp]),
+    "ka_ctx_set_report_brokers": (_i32, [_vp, _i32, _vp]),
+    "ka_plan_last": (_i32, [_vp, _vp, _vp, _vp]),
     "ka_ctx_counter_slots": (_i32, [_vp]),
     "ka_ctx_get_counters": (_i32, [_vp, _vp]),
     "ka_ctx_set_counters": (_i32, [_vp, _vp]),

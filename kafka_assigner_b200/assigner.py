@@ -14,7 +14,12 @@ import ctypes
 import numpy as np
 
 from . import _native
-from ._native import KaStatus
+from ._native import KaPlanTotals, KaStatus
+
+# movement plan (ka_plan_last): row classes and the columns of Solver.last_plan()'s per-broker table
+ROW_UNCHANGED, ROW_REORDERED, ROW_MOVED = 0, 1, 2
+PLAN_COLUMNS = ("replicas_before", "replicas_after", "replicas_in", "replicas_out",
+                "leaders_before", "leaders_after", "leaders_in", "leaders_out")
 
 
 class IllegalStateException(Exception):
@@ -71,6 +76,8 @@ class Solver:
         self.device = device
         self.N = 0
         self.broker_id = None
+        self.report_ids = None   # set_report_brokers(); None = the live broker table
+        self._last_rows = None   # rows of the last solve issued through this object (None: no solve, or the split API)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -158,6 +165,7 @@ class Solver:
         if out_len is None:
             out_len = np.zeros((T, P), dtype=np.int32)
         st = KaStatus()
+        self._last_rows = T * P
         self._L.ka_solve_dense(self._h, T, _ptr(th), P, RF, _ptr(cur), int(desired_rf), int(out_stride), _ptr(out_len),
                                _ptr(out), ctypes.byref(st))
         if check:
@@ -172,9 +180,12 @@ class Solver:
         name_off[1:] = np.cumsum([len(e) for e in enc])
         return np.frombuffer(b"".join(enc) or b"\0", dtype=np.uint8), name_off
 
-    def solve_dense_json(self, topic_names, topic_hash, cur, desired_rf=-1, json_buf=None, check=True, names_slab=None):
+    def solve_dense_json(self, topic_names, topic_hash, cur, desired_rf=-1, json_buf=None, check=True, names_slab=None,
+                         changed_only=False):
         """Solve + emit the reassignment JSON on the device (KAG:169-186); returns (bytes-like view of the text, status).
-        json_buf: optional writable uint8 numpy array (pinned memory for full PCIe speed); names_slab: marshal_names() result."""
+        json_buf: optional writable uint8 numpy array (pinned memory for full PCIe speed); names_slab: marshal_names() result.
+        changed_only: list only the partitions whose replica list changes (ka_solve_dense_json_changed); same format, and
+        '{"partitions":[],"version":1}' when nothing changes."""
         cur = np.ascontiguousarray(cur, dtype=np.int32)
         T, P, RF = cur.shape
         th = np.ascontiguousarray(topic_hash, dtype=np.int32)
@@ -185,8 +196,10 @@ class Solver:
             json_buf = np.empty(cap, dtype=np.uint8)
         nbytes = ctypes.c_int64(0)
         st = KaStatus()
-        self._L.ka_solve_dense_json(self._h, T, _ptr(th), P, RF, _ptr(cur), int(desired_rf), _ptr(names), _ptr(name_off),
-                                    _ptr(json_buf), int(json_buf.size), ctypes.byref(nbytes), ctypes.byref(st))
+        self._last_rows = T * P
+        fn = self._L.ka_solve_dense_json_changed if changed_only else self._L.ka_solve_dense_json
+        fn(self._h, T, _ptr(th), P, RF, _ptr(cur), int(desired_rf), _ptr(names), _ptr(name_off), _ptr(json_buf),
+           int(json_buf.size), ctypes.byref(nbytes), ctypes.byref(st))
         if check:
             raise_for_status(st, topic_names)
         return json_buf[:nbytes.value], st
@@ -202,6 +215,7 @@ class Solver:
         out = np.full((Q, out_stride), -1, dtype=np.int32)
         out_len = np.zeros(Q, dtype=np.int32)
         st = KaStatus()
+        self._last_rows = Q
         self._L.ka_solve(self._h, len(th), _ptr(th), _ptr(part_off), _ptr(part_id), _ptr(rep_off), _ptr(cur_broker),
                          int(desired_rf), int(out_stride), _ptr(out_len), _ptr(out), ctypes.byref(st))
         if check:
@@ -210,8 +224,10 @@ class Solver:
 
     def solve_dense_device(self, T, d_topic_hash, P, RF, d_cur, desired_rf, out_stride, d_out_len, d_out, stream=0,
                            sync=True):
-        """Device-pointer form (ints from tensor.data_ptr()); returns KaStatus when sync else None."""
+        """Device-pointer form (ints from tensor.data_ptr()); returns KaStatus when sync else None. last_plan() after this
+        reads the caller's d_cur / d_out / d_out_len: keep them alive and unchanged until then."""
         st = KaStatus()
+        self._last_rows = int(T) * int(P)
         rc = self._L.ka_solve_dense_device(self._h, int(T), ctypes.c_void_p(d_topic_hash), int(P), int(RF),
                                            ctypes.c_void_p(d_cur), int(desired_rf), int(out_stride),
                                            ctypes.c_void_p(d_out_len) if d_out_len else None, ctypes.c_void_p(d_out),
@@ -225,6 +241,7 @@ class Solver:
 
     def stage_dense_device(self, T, d_topic_hash, P, RF, d_cur, desired_rf, out_stride, stream=0):
         """Context-free stage (KAS:65-200) of a topic block — shards across GPUs."""
+        self._last_rows = None
         rc = self._L.ka_stage_dense_device(self._h, int(T), ctypes.c_void_p(d_topic_hash), int(P), int(RF),
                                            ctypes.c_void_p(d_cur), int(desired_rf), int(out_stride),
                                            ctypes.c_void_p(stream) if stream else None)
@@ -286,6 +303,39 @@ class Solver:
         rc = self._L.ka_ctx_import_counters_device(self._h, ctypes.c_void_p(d_ptr), ctypes.c_void_p(stream) if stream else None)
         if rc:
             raise KassignError(rc)
+
+    # -- movement plan ---------------------------------------------------------------------------
+    def set_report_brokers(self, ids=None):
+        """Broker ids that last_plan() reports one by one (strictly ascending after sorting, at most 65534); every other id
+        falls into the extra 'other' row. None or empty: the live broker table (decommissioned brokers land in 'other')."""
+        b = np.zeros(0, dtype=np.int32) if ids is None else np.ascontiguousarray(np.sort(np.asarray(ids, dtype=np.int32)))
+        rc = self._L.ka_ctx_set_report_brokers(self._h, len(b), _ptr(b) if len(b) else None)
+        if rc:
+            raise KassignError(rc, "ka_ctx_set_report_brokers")
+        self.report_ids = b if len(b) else None
+
+    def last_plan(self, row_class=False):
+        """Movement plan of the last successful solve, computed on the device (ka_plan_last).
+
+        Returns (totals, broker_ids, broker_stats, row_class):
+          totals        dict rows, rows_reordered, rows_moved, replicas_added, replicas_dropped, leaders_changed
+          broker_ids    int32 [M]: the report ids (set_report_brokers, default the live broker table)
+          broker_stats  uint32 [M + 1, 8]: row i for broker_ids[i], row M for every other id; columns PLAN_COLUMNS =
+                        replicas_before, replicas_after, replicas_in (copied to the broker), replicas_out (removed from it),
+                        leaders_before, leaders_after, leaders_in (leadership gained), leaders_out (leadership lost)
+          row_class     uint8 [rows] ROW_UNCHANGED / ROW_REORDERED (same brokers, new order) / ROW_MOVED (brokers differ), or
+                        None unless row_class=True
+        """
+        ids = self.report_ids if self.report_ids is not None else (self.broker_id if self.broker_id is not None
+                                                                   else np.zeros(0, dtype=np.int32))
+        stats = np.zeros((len(ids) + 1, len(PLAN_COLUMNS)), dtype=np.uint32)
+        cls = np.zeros(self._last_rows or 0, dtype=np.uint8) if row_class else None
+        tot = KaPlanTotals()
+        rc = self._L.ka_plan_last(self._h, _ptr(cls) if row_class and self._last_rows else None, _ptr(stats), ctypes.byref(tot))
+        if rc:
+            raise KassignError(rc, "ka_plan_last: no successful solve to plan")
+        totals = {name: int(getattr(tot, name)) for name, _ in KaPlanTotals._fields_}
+        return totals, ids.copy(), stats, cls
 
     def solve_cluster(self, cluster, check=True):
         """The KAG:172-184 loop for a synth.Cluster: all topics in order through this Context."""

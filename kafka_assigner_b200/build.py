@@ -7,7 +7,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB = os.path.join(CSRC, "libkassign.so")
 SOURCES = ["kassign.cu"]
-HEADERS = ["kassign_common.cuh", "kassign_stage.cuh", "kassign_order.cuh", os.path.join("..", "..", "include", "kassign.h")]
+HEADERS = ["kassign_common.cuh", "kassign_stage.cuh", "kassign_order.cuh", "kassign_json.cuh", "kassign_plan.cuh",
+           os.path.join("..", "..", "include", "kassign.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 

@@ -1,10 +1,12 @@
-// kassign.cu — C ABI (include/kassign.h) over the sm_100a kernels in kassign_stage.cuh / kassign_order.cuh / kassign_json.cuh.
+// kassign.cu — C ABI (include/kassign.h) over the sm_100a kernels in kassign_stage.cuh / kassign_order.cuh / kassign_json.cuh /
+// kassign_plan.cuh.
 //
 // Reference boundary: KafkaTopicAssigner.generateAssignment (KafkaTopicAssigner.java:42-72) batched over
 // the topic loop of KafkaAssignmentGenerator.java:172-184. No CPU fallback exists in this library.
 #include "kassign_stage.cuh"
 #include "kassign_order.cuh"
 #include "kassign_json.cuh"
+#include "kassign_plan.cuh"
 
 #include <algorithm>
 #include <climits>
@@ -26,6 +28,7 @@ constexpr int KA_SM_COUNT_FALLBACK = 148;
 constexpr size_t KA_SMEM_BUDGET = 200 * 1024;   // per-CTA dynamic smem we allow ourselves (of 227 KB)
 constexpr uint32_t KA_LUT_SMEM_MAX_RANGE = 32768;
 constexpr uint32_t KA_LUT_GLOBAL_MAX_RANGE = 1u << 25;
+constexpr size_t KA_PLAN_SMEM_BUDGET = 112 * 1024;  // plan kernel: id LUT + private per-broker columns, two CTAs per SM
 
 struct DevBuf {
     void* p = nullptr;
@@ -119,6 +122,14 @@ struct ka_ctx {
     const int32_t* last_part_id = nullptr;  // host pointer (ragged API) for status translation
     const int64_t* last_part_off = nullptr;
     ka_status last{};
+    // movement plan (ka_plan_last): rows of the last solve, still resident; report-id table (rep_M == 0: the live table)
+    bool plan_valid = false;
+    KaRows plan_rows{};
+    int64_t plan_Q = 0;
+    int rep_M = 0, rep_mode = KA_LUT_SMEM, rep_min_id = 0;
+    uint32_t rep_range = 0;
+    DevBuf d_rep_lut, d_rep_ids, d_plan_tot, d_plan_stats, d_plan_class;
+    DevBuf d_sel, d_sel_mask, d_sel_blockcnt, d_sel_state;  // changed-row compaction of ka_solve_dense_json_changed
 };
 
 namespace {
@@ -145,6 +156,31 @@ int set_status(ka_status* st, int code, int topic = -1, int part = -1, int a = 0
 }
 
 inline size_t align16(size_t v) { return (v + 15) & ~size_t(15); }
+
+// Id -> index table of n strictly ascending ids (ka_id_index): a 16-bit LUT over the id range, staged into shared memory up
+// to KA_LUT_SMEM_MAX_RANGE ids and read from global memory (L2) up to KA_LUT_GLOBAL_MAX_RANGE; beyond that a binary search
+// over the ids. Used by the live broker table and by the report-id table of the movement plan.
+struct IdLut {
+    int mode = KA_LUT_SMEM;
+    int min_id = 0;
+    uint32_t range = 0;
+    std::vector<uint16_t> lut;  // [range rounded up to 16 bytes], KA_DEAD where no id; empty for KA_LUT_BSEARCH
+};
+
+IdLut make_id_lut(int n, const int32_t* ids) {
+    IdLut t;
+    t.min_id = n > 0 ? ids[0] : 0;
+    const uint64_t range64 = n > 0 ? (uint64_t)((int64_t)ids[n - 1] - (int64_t)ids[0]) + 1 : 0;
+    if (range64 > KA_LUT_GLOBAL_MAX_RANGE) {
+        t.mode = KA_LUT_BSEARCH;
+        return t;
+    }
+    t.mode = range64 <= KA_LUT_SMEM_MAX_RANGE ? KA_LUT_SMEM : KA_LUT_GLOBAL;
+    t.range = (uint32_t)range64;
+    t.lut.assign(align16((size_t)std::max<uint64_t>(range64, 1) * 2) / 2, (uint16_t)KA_DEAD);
+    for (int i = 0; i < n; ++i) t.lut[(size_t)((int64_t)ids[i] - t.min_id)] = (uint16_t)i;
+    return t;
+}
 
 // download current device counters into ctx->parked keyed by id
 int park_counters(ka_ctx* c) {
@@ -246,6 +282,18 @@ int make_plan(ka_ctx* c, int64_t Q, int S, int Pmax, int64_t capmax, bool ragged
 template <typename K>
 cudaError_t allow_smem(K kernel, size_t bytes) {
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
+
+template <int SM, bool SHIST>
+cudaError_t launch_plan(ka_ctx* c, cudaStream_t s, const KaPlanParams& p, size_t smem) {
+    auto kern = ka_plan_kernel<SM, SHIST>;
+    cudaError_t e = allow_smem(kern, smem);
+    if (e != cudaSuccess) return e;
+    int occ = 1;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 512, smem)) != cudaSuccess) return e;
+    const int64_t grid = std::min<int64_t>((p.Q + 511) / 512, (int64_t)std::max(occ, 1) * c->sm_count);
+    kern<<<(unsigned)grid, 512, smem, s>>>(p);
+    return cudaGetLastError();
 }
 
 // One contiguous block of topics of a dense or ragged problem, with every device pointer already offset to the block.
@@ -429,6 +477,8 @@ struct JsonJob {
     int32_t* d_out_len;
     int S;
     int blocks = 0;
+    bool changed_only = false;  // ka_solve_dense_json_changed: text of the rows whose class is not UNCHANGED only
+    KaRows rows{};              // changed_only: current + new lists of the run (ka_row_diff)
 };
 namespace {
 
@@ -458,10 +508,33 @@ int enq_json_rows(ka_ctx* c, cudaStream_t s_done, int64_t row0, int64_t rows, in
     p.first = first;
     p.last = last;
     const int nblocks = (int)((rows + 255) / 256);
-    if (nblocks > 0) ka_json_len_kernel<<<nblocks, 256, 0, c->sj>>>(p);
-    ka_json_scan_kernel<<<1, 1024, 0, c->sj>>>(p, nblocks);
-    KA_CUDA(allow_smem(ka_json_write_kernel, KA_JSON_SMEM_BYTES + 16));
-    ka_json_write_kernel<<<std::max(nblocks, 1), 256, KA_JSON_SMEM_BYTES + 16, c->sj>>>(p);
+    if (jj->changed_only) {
+        // compact the fragment's changed rows (fragment-relative, row order) into sel; the count stays on the device, so the
+        // text kernels below cover every row of the fragment and their blocks beyond the count write nothing
+        uint32_t* mask = c->d_sel_mask.as<uint32_t>() + (size_t)(row0 / 256 + k) * 8;
+        uint32_t* blockcnt = c->d_sel_blockcnt.as<uint32_t>() + row0 / 256 + k;
+        uint32_t* state = c->d_sel_state.as<uint32_t>();   // [0] rows kept so far, then {before, count} per fragment
+        uint32_t* sel = c->d_sel.as<uint32_t>() + row0;
+        if (nblocks > 0) {
+            if (jj->S <= 3) ka_changed_flag_kernel<3><<<nblocks, 256, 0, c->sj>>>(jj->rows, row0, (uint32_t)rows, mask, blockcnt);
+            else ka_changed_flag_kernel<8><<<nblocks, 256, 0, c->sj>>>(jj->rows, row0, (uint32_t)rows, mask, blockcnt);
+        }
+        ka_changed_scan_kernel<<<1, 1024, 0, c->sj>>>(blockcnt, nblocks, state, state + 1 + 2 * k);
+        if (nblocks > 0) ka_changed_scatter_kernel<<<nblocks, 256, 0, c->sj>>>(mask, blockcnt, (uint32_t)rows, sel);
+        KA_CUDA(cudaGetLastError());
+        c->launches += nblocks > 0 ? 3 : 1;
+        p.sel = sel;
+        p.sel_state = state + 1 + 2 * k;
+        if (nblocks > 0) ka_json_len_kernel<true><<<nblocks, 256, 0, c->sj>>>(p);
+        ka_json_scan_kernel<<<1, 1024, 0, c->sj>>>(p, nblocks);
+        KA_CUDA(allow_smem(ka_json_write_kernel<true>, KA_JSON_SMEM_BYTES + 16));
+        ka_json_write_kernel<true><<<std::max(nblocks, 1), 256, KA_JSON_SMEM_BYTES + 16, c->sj>>>(p);
+    } else {
+        if (nblocks > 0) ka_json_len_kernel<false><<<nblocks, 256, 0, c->sj>>>(p);
+        ka_json_scan_kernel<<<1, 1024, 0, c->sj>>>(p, nblocks);
+        KA_CUDA(allow_smem(ka_json_write_kernel<false>, KA_JSON_SMEM_BYTES + 16));
+        ka_json_write_kernel<false><<<std::max(nblocks, 1), 256, KA_JSON_SMEM_BYTES + 16, c->sj>>>(p);
+    }
     KA_CUDA(cudaGetLastError());
     KA_CUDA(cudaMemcpyAsync(c->h_frag + 2 * k, p.frag, 16, cudaMemcpyDeviceToHost, c->sj));
     KA_CUDA(cudaEventRecord(c->ev_json_scan[k], c->sj));
@@ -866,6 +939,9 @@ void ka_ctx_destroy(ka_ctx* c) {
     for (auto& e : c->ev_json_in) if (e) cudaEventDestroy(e);
     for (auto& e : c->ev_json_scan) if (e) cudaEventDestroy(e);
     for (DevBuf* b : {&c->d_json, &c->d_names, &c->d_name_off, &c->d_json_rowlen, &c->d_json_blocksum, &c->d_json_state}) b->release();
+    for (DevBuf* b : {&c->d_rep_lut, &c->d_rep_ids, &c->d_plan_tot, &c->d_plan_stats, &c->d_plan_class, &c->d_sel, &c->d_sel_mask,
+                      &c->d_sel_blockcnt, &c->d_sel_state})
+        b->release();
     if (c->ev_chain_in) cudaEventDestroy(c->ev_chain_in);
     if (c->ev_out_done) cudaEventDestroy(c->ev_out_done);
     for (auto& e : c->ev_b1) if (e) cudaEventDestroy(e);
@@ -906,8 +982,6 @@ int32_t ka_ctx_set_brokers(ka_ctx* c, int32_t N, const int32_t* broker_id, const
     c->N = N;
     c->broker_id.assign(broker_id, broker_id + N);
     c->broker_rack.assign(broker_rack, broker_rack + N);
-    c->min_id = N > 0 ? broker_id[0] : 0;
-    const uint64_t range64 = N > 0 ? (uint64_t)((int64_t)broker_id[N - 1] - (int64_t)broker_id[0]) + 1 : 0;
     const size_t npad = align16((size_t)std::max(N, 1) * 2) / 2;  // uint16 elements, 16B multiple
     // compact rack ids in order of first appearance (rack identity is all that matters, KAS:90-94)
     std::vector<uint16_t> rackc(std::max(N, 1), 0);
@@ -921,31 +995,22 @@ int32_t ka_ctx_set_brokers(ka_ctx* c, int32_t N, const int32_t* broker_id, const
         c->R = (int)seen.size();
     }
     std::vector<uint16_t> blob;
-    size_t lut_elems = 0;
-    if (range64 <= KA_LUT_SMEM_MAX_RANGE) {
-        c->lut_mode = KA_LUT_SMEM;
-        c->range = (uint32_t)range64;
-        lut_elems = align16((size_t)std::max<uint64_t>(range64, 1) * 2) / 2;
-    } else if (range64 <= KA_LUT_GLOBAL_MAX_RANGE) {
-        c->lut_mode = KA_LUT_GLOBAL;
-        c->range = (uint32_t)range64;
-        std::vector<uint16_t> g((size_t)range64, (uint16_t)KA_DEAD);
-        for (int i = 0; i < N; ++i) g[(size_t)((int64_t)broker_id[i] - c->min_id)] = (uint16_t)i;
-        KA_CUDA(c->d_glut.reserve(g.size() * 2));
-        KA_CUDA(cudaMemcpy(c->d_glut.p, g.data(), g.size() * 2, cudaMemcpyHostToDevice));
-    } else {
-        c->lut_mode = KA_LUT_BSEARCH;
-        c->range = 0;
+    const IdLut lut = make_id_lut(N, broker_id);
+    c->lut_mode = lut.mode;
+    c->min_id = lut.min_id;
+    c->range = lut.range;
+    const size_t lut_elems = lut.mode == KA_LUT_SMEM ? lut.lut.size() : 0;  // the shared-memory LUT travels in the blob
+    if (lut.mode == KA_LUT_GLOBAL) {
+        KA_CUDA(c->d_glut.reserve(lut.lut.size() * 2));
+        KA_CUDA(cudaMemcpy(c->d_glut.p, lut.lut.data(), lut.lut.size() * 2, cudaMemcpyHostToDevice));
     }
     const size_t roff_elems = align16((size_t)(c->R + 1) * 2) / 2;
     c->lut_off = (int)npad;
     c->roff_off = (int)(npad + lut_elems);
     c->memb_off = (int)(npad + lut_elems + roff_elems);
     blob.assign(npad + lut_elems + roff_elems + npad, (uint16_t)KA_DEAD);
-    for (int i = 0; i < N; ++i) {
-        blob[i] = rackc[i];
-        if (c->lut_mode == KA_LUT_SMEM) blob[npad + (size_t)((int64_t)broker_id[i] - c->min_id)] = (uint16_t)i;
-    }
+    for (int i = 0; i < N; ++i) blob[i] = rackc[i];
+    std::copy(lut.lut.begin(), lut.lut.begin() + lut_elems, blob.begin() + npad);
     {   // rack member lists (CSR): sorted indices ascending inside each rack
         std::vector<int> cntr(c->R + 1, 0);
         for (int i = 0; i < N; ++i) cntr[rackc[i] + 1]++;
@@ -1041,9 +1106,17 @@ static int validate_dense(ka_ctx* c, int32_t T, int32_t P, int32_t RF, int32_t d
     return KA_OK;
 }
 
+// Rows of a dense solve as the movement plan reads them; recorded when the solve is enqueued (ka_plan_last runs on them).
+static void keep_dense_rows(ka_ctx* c, int64_t Q, const int32_t* d_cur, int RF, int32_t* d_out, int32_t* d_out_len, int S, int desired_rf) {
+    c->plan_rows = KaRows{d_cur, nullptr, RF, d_out, d_out_len, S, desired_rf >= 0 ? desired_rf : RF};
+    c->plan_Q = Q;
+    c->plan_valid = true;
+}
+
 int32_t ka_solve_dense_device(ka_ctx* c, int32_t T, const int32_t* d_topic_hash, int32_t P, int32_t RF,
                               const int32_t* d_cur_broker, int32_t desired_rf, int32_t out_stride,
                               int32_t* d_out_len, int32_t* d_out_broker, void* stream, ka_status* st) {
+    if (c) c->plan_valid = false;
     int rc = validate_dense(c, T, P, RF, desired_rf, out_stride, st);
     if (rc != KA_OK) return rc;
     if (cudaSetDevice(c->device) != cudaSuccess) return set_status(st, KA_ERR_CUDA);
@@ -1056,6 +1129,7 @@ int32_t ka_solve_dense_device(ka_ctx* c, int32_t T, const int32_t* d_topic_hash,
     rc = run_dense(c, s, T, P, RF, desired_rf, out_stride, nullptr, nullptr, const_cast<int32_t*>(d_topic_hash),
                    const_cast<int32_t*>(d_cur_broker), d_out_broker, d_out_len, nullptr, nullptr, st);
     if (rc != KA_OK) { if (st && st->code != rc) set_status(st, rc); return rc; }
+    keep_dense_rows(c, (int64_t)T * P, d_cur_broker, RF, d_out_broker, d_out_len, out_stride, desired_rf);
     c->last_stream = s;
     c->pending_status = true;
     if (st) return finish_status(c, s, st);
@@ -1064,6 +1138,7 @@ int32_t ka_solve_dense_device(ka_ctx* c, int32_t T, const int32_t* d_topic_hash,
 
 int32_t ka_stage_dense_device(ka_ctx* c, int32_t T, const int32_t* d_topic_hash, int32_t P, int32_t RF,
                               const int32_t* d_cur_broker, int32_t desired_rf, int32_t out_stride, void* stream) {
+    if (c) c->plan_valid = false;   // the split stage / order / emit solve has no movement plan
     ka_status lst;
     int rc = validate_dense(c, T, P, RF, desired_rf, out_stride, &lst);
     if (rc != KA_OK) return rc;
@@ -1194,6 +1269,7 @@ int32_t ka_ctx_set_topic_base(ka_ctx* c, int32_t topic_base) {
 int32_t ka_solve_dense(ka_ctx* c, int32_t T, const int32_t* topic_hash, int32_t P, int32_t RF,
                        const int32_t* cur_broker, int32_t desired_rf, int32_t out_stride,
                        int32_t* out_len, int32_t* out_broker, ka_status* st) {
+    if (c) c->plan_valid = false;
     int rc = validate_dense(c, T, P, RF, desired_rf, out_stride, st);
     if (rc != KA_OK) return rc;
     if (cudaSetDevice(c->device) != cudaSuccess) return set_status(st, KA_ERR_CUDA);
@@ -1212,17 +1288,21 @@ int32_t ka_solve_dense(ka_ctx* c, int32_t T, const int32_t* topic_hash, int32_t 
     rc = run_dense(c, s, T, P, RF, desired_rf, out_stride, topic_hash, cur_broker, c->d_hash.as<int32_t>(), c->d_cur.as<int32_t>(),
                    c->d_out.as<int32_t>(), c->d_out_len.as<int32_t>(), out_broker, out_len, st);
     if (rc != KA_OK) { if (st && st->code != rc) set_status(st, rc); return rc; }
+    keep_dense_rows(c, Q, c->d_cur.as<int32_t>(), RF, c->d_out.as<int32_t>(), c->d_out_len.as<int32_t>(), out_stride, desired_rf);
     c->last_stream = s;
     c->pending_status = true;
     ka_status local;
     return finish_status(c, s, st ? st : &local);
 }
 
-int32_t ka_solve_dense_json(ka_ctx* c, int32_t T, const int32_t* topic_hash, int32_t P, int32_t RF, const int32_t* cur_broker,
-                            int32_t desired_rf, const char* names, const int64_t* name_off, char* json, int64_t json_cap,
-                            int64_t* json_bytes, ka_status* st) {
+}  // extern "C"
+
+static int32_t solve_dense_json(ka_ctx* c, int32_t T, const int32_t* topic_hash, int32_t P, int32_t RF, const int32_t* cur_broker,
+                                int32_t desired_rf, const char* names, const int64_t* name_off, char* json, int64_t json_cap,
+                                int64_t* json_bytes, ka_status* st, bool changed_only) {
     const int S = std::max(std::max(RF, desired_rf), 1);
     if (json_bytes) *json_bytes = 0;
+    if (c) c->plan_valid = false;
     int rc = validate_dense(c, T, P, RF, desired_rf, S, st);
     if (rc != KA_OK) return rc;
     const int64_t Q = (int64_t)T * P, R = Q * RF;
@@ -1250,6 +1330,17 @@ int32_t ka_solve_dense_json(ka_ctx* c, int32_t T, const int32_t* topic_hash, int
     if (name_bytes > 0) KA_CUDA(cudaMemcpyAsync(c->d_names.p, names, (size_t)name_bytes, cudaMemcpyHostToDevice, c->sj));
     if (T > 0) KA_CUDA(cudaMemcpyAsync(c->d_name_off.p, name_off, (size_t)(T + 1) * 8, cudaMemcpyHostToDevice, c->sj));
     JsonJob job{c->d_out.as<int32_t>(), c->d_out_len.as<int32_t>(), S, 0};
+    if (changed_only) {
+        const size_t frag_blocks = (size_t)(Q / 256 + 2 * KA_MAX_CHAIN_EVENTS);
+        KA_CUDA(c->d_sel.reserve((size_t)std::max<int64_t>(Q, 1) * 4));
+        KA_CUDA(c->d_sel_mask.reserve(frag_blocks * 8 * 4));
+        KA_CUDA(c->d_sel_blockcnt.reserve(frag_blocks * 4));
+        KA_CUDA(c->d_sel_state.reserve((1 + 2 * KA_MAX_CHAIN_EVENTS) * 4));
+        KA_CUDA(cudaMemsetAsync(c->d_sel_state.p, 0, (1 + 2 * KA_MAX_CHAIN_EVENTS) * 4, c->sj));
+        job.changed_only = true;
+        job.rows = KaRows{c->d_cur.as<int32_t>(), nullptr, RF, c->d_out.as<int32_t>(), c->d_out_len.as<int32_t>(), S,
+                          desired_rf >= 0 ? desired_rf : RF};
+    }
     c->json_job = &job;
     c->last_part_id = nullptr;
     c->last_part_off = nullptr;
@@ -1260,6 +1351,7 @@ int32_t ka_solve_dense_json(ka_ctx* c, int32_t T, const int32_t* topic_hash, int
                             : KA_ERR_BAD_ARG;
     c->json_job = nullptr;
     if (rc != KA_OK) { if (st && st->code != rc) set_status(st, rc); cudaStreamSynchronize(c->sj); return rc; }
+    keep_dense_rows(c, Q, c->d_cur.as<int32_t>(), RF, c->d_out.as<int32_t>(), c->d_out_len.as<int32_t>(), S, desired_rf);
     c->last_stream = s;
     c->pending_status = true;
     // every block is enqueued; stream the fragments out as their sizes become known (later blocks are still in the chains)
@@ -1275,9 +1367,26 @@ int32_t ka_solve_dense_json(ka_ctx* c, int32_t T, const int32_t* topic_hash, int
     KA_CUDA(cudaStreamSynchronize(c->sj));
     ka_status local;
     rc = finish_status(c, s, st ? st : &local);
-    if (rc == KA_OK && overflow) return set_status(st, KA_ERR_LIMIT, -1, -1, (int)std::min<int64_t>(json_cap, INT_MAX));
+    if (rc == KA_OK && overflow) {
+        c->plan_valid = false;
+        return set_status(st, KA_ERR_LIMIT, -1, -1, (int)std::min<int64_t>(json_cap, INT_MAX));
+    }
     if (json_bytes) *json_bytes = rc == KA_OK ? total : 0;
     return rc;
+}
+
+extern "C" {
+
+int32_t ka_solve_dense_json(ka_ctx* c, int32_t T, const int32_t* topic_hash, int32_t P, int32_t RF, const int32_t* cur_broker,
+                            int32_t desired_rf, const char* names, const int64_t* name_off, char* json, int64_t json_cap,
+                            int64_t* json_bytes, ka_status* st) {
+    return solve_dense_json(c, T, topic_hash, P, RF, cur_broker, desired_rf, names, name_off, json, json_cap, json_bytes, st, false);
+}
+
+int32_t ka_solve_dense_json_changed(ka_ctx* c, int32_t T, const int32_t* topic_hash, int32_t P, int32_t RF, const int32_t* cur_broker,
+                                    int32_t desired_rf, const char* names, const int64_t* name_off, char* json, int64_t json_cap,
+                                    int64_t* json_bytes, ka_status* st) {
+    return solve_dense_json(c, T, topic_hash, P, RF, cur_broker, desired_rf, names, name_off, json, json_cap, json_bytes, st, true);
 }
 
 int32_t ka_solve(ka_ctx* c, int32_t T, const int32_t* topic_hash, const int64_t* part_off,
@@ -1286,6 +1395,7 @@ int32_t ka_solve(ka_ctx* c, int32_t T, const int32_t* topic_hash, const int64_t*
                  ka_status* st) {
     set_status(st, KA_OK);
     if (!c) return set_status(st, KA_ERR_NO_DEVICE);
+    c->plan_valid = false;
     if (T < 0 || (T > 0 && (!topic_hash || !part_off))) return set_status(st, KA_ERR_BAD_ARG);
     const int S = out_stride;
     if (S < 1 || S > KA_MAX_SLOTS) return set_status(st, KA_ERR_LIMIT, -1, -1, S);
@@ -1368,6 +1478,10 @@ int32_t ka_solve(ka_ctx* c, int32_t T, const int32_t* topic_hash, const int64_t*
     }
     if ((rc = enq_flags_readback(c, s)) != KA_OK) return set_status(st, rc);
     if (c->timing) { KA_CUDA(cudaEventRecord(c->ev[5], s)); c->ev_valid = true; }
+    c->plan_rows = KaRows{c->d_cur.as<int32_t>(), c->d_rep_off.as<int64_t>(), 0, c->d_out.as<int32_t>(), c->d_out_len.as<int32_t>(), S,
+                          desired_rf};
+    c->plan_Q = Q;
+    c->plan_valid = true;
     c->last_stream = s;
     c->pending_status = true;
     ka_status local;
@@ -1375,6 +1489,82 @@ int32_t ka_solve(ka_ctx* c, int32_t T, const int32_t* topic_hash, const int64_t*
     c->last_part_id = nullptr;
     c->last_part_off = nullptr;
     return rc;
+}
+
+int32_t ka_ctx_set_report_brokers(ka_ctx* c, int32_t M, const int32_t* ids) {
+    if (!c) return KA_ERR_NO_DEVICE;
+    if (M < 0 || M > 65534 || (M > 0 && !ids)) return KA_ERR_BAD_ARG;   // bucket M ("other") must stay below KA_DEAD
+    for (int i = 1; i < M; ++i)
+        if (ids[i] <= ids[i - 1]) return KA_ERR_BAD_ARG;   // ascending, distinct
+    KA_CUDA(cudaSetDevice(c->device));
+    if (c->pending_status) finish_status(c, c->last_stream, nullptr);
+    c->rep_M = 0;
+    if (M == 0) return KA_OK;
+    const IdLut lut = make_id_lut(M, ids);
+    if (!lut.lut.empty()) {
+        KA_CUDA(c->d_rep_lut.reserve(lut.lut.size() * 2));
+        KA_CUDA(cudaMemcpy(c->d_rep_lut.p, lut.lut.data(), lut.lut.size() * 2, cudaMemcpyHostToDevice));
+    }
+    KA_CUDA(c->d_rep_ids.reserve((size_t)M * 4));
+    KA_CUDA(cudaMemcpy(c->d_rep_ids.p, ids, (size_t)M * 4, cudaMemcpyHostToDevice));
+    c->rep_mode = lut.mode;
+    c->rep_min_id = lut.min_id;
+    c->rep_range = lut.range;
+    c->rep_M = M;
+    return KA_OK;
+}
+
+int32_t ka_plan_last(ka_ctx* c, uint8_t* row_class, uint32_t* broker_stats, ka_plan_totals* totals) {
+    if (!c) return KA_ERR_NO_DEVICE;
+    KA_CUDA(cudaSetDevice(c->device));
+    if (c->pending_status) finish_status(c, c->last_stream, nullptr);
+    if (!c->plan_valid || c->last.code != KA_OK) return KA_ERR_BAD_ARG;
+    KaPlanParams p{};
+    p.rows = c->plan_rows;
+    p.Q = c->plan_Q;
+    if (c->rep_M > 0) {
+        p.lut_mode = c->rep_mode;
+        p.min_id = c->rep_min_id;
+        p.range = c->rep_range;
+        p.glut = c->d_rep_lut.as<uint16_t>();
+        p.broker_id = c->d_rep_ids.as<int32_t>();
+        p.N = c->rep_M;
+    } else {   // the live broker table, through the lookup kernel A uses
+        p.lut_mode = c->lut_mode;
+        p.min_id = c->min_id;
+        p.range = c->range;
+        p.glut = c->lut_mode == KA_LUT_SMEM ? c->d_blob.as<uint16_t>() + c->lut_off : c->d_glut.as<uint16_t>();
+        p.broker_id = c->d_broker_id.as<int32_t>();
+        p.N = c->N;
+    }
+    p.lut_bytes = p.lut_mode == KA_LUT_SMEM ? (int)align16((size_t)p.range * 2) : 0;
+    const size_t ncol = (size_t)(p.N + 1) * KA_PLAN_COLS;
+    const bool shist = p.lut_bytes + ncol * 4 <= KA_PLAN_SMEM_BUDGET;
+    const size_t smem = p.lut_bytes + (shist ? ncol * 4 : 0);
+    cudaStream_t s = c->stream;
+    KA_CUDA(c->d_plan_tot.reserve(KA_PLAN_TOTALS * 8));
+    KA_CUDA(c->d_plan_stats.reserve(ncol * 4));
+    KA_CUDA(cudaMemsetAsync(c->d_plan_tot.p, 0, KA_PLAN_TOTALS * 8, s));
+    KA_CUDA(cudaMemsetAsync(c->d_plan_stats.p, 0, ncol * 4, s));
+    if (row_class && p.Q > 0) {
+        KA_CUDA(c->d_plan_class.reserve((size_t)p.Q));
+        p.row_class = c->d_plan_class.as<uint8_t>();
+    }
+    p.stats = c->d_plan_stats.as<uint32_t>();
+    p.totals = c->d_plan_tot.as<unsigned long long>();
+    if (p.Q > 0) {
+        const bool wide = p.rows.S > 3;
+        KA_CUDA(wide ? (shist ? launch_plan<8, true>(c, s, p, smem) : launch_plan<8, false>(c, s, p, smem))
+                     : (shist ? launch_plan<3, true>(c, s, p, smem) : launch_plan<3, false>(c, s, p, smem)));
+        c->launches++;
+    }
+    int64_t tot[KA_PLAN_TOTALS];
+    KA_CUDA(cudaMemcpyAsync(tot, c->d_plan_tot.p, sizeof(tot), cudaMemcpyDeviceToHost, s));
+    if (broker_stats) KA_CUDA(cudaMemcpyAsync(broker_stats, c->d_plan_stats.p, ncol * 4, cudaMemcpyDeviceToHost, s));
+    if (p.row_class) KA_CUDA(cudaMemcpyAsync(row_class, p.row_class, (size_t)p.Q, cudaMemcpyDeviceToHost, s));
+    KA_CUDA(cudaStreamSynchronize(s));
+    if (totals) *totals = ka_plan_totals{tot[0], tot[1], tot[2], tot[3], tot[4], tot[5]};
+    return KA_OK;
 }
 
 }  // extern "C"

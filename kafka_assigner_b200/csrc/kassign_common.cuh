@@ -84,6 +84,29 @@ __device__ __forceinline__ int4 ka_ldg_stream_v4(const int4* p) {
     return r;
 }
 
+// Broker id -> index in an ascending id table, KA_DEAD when absent. The host picks the mode from the id range when it builds
+// the table (make_id_lut in kassign.cu): a 16-bit LUT in shared memory (`lut`), the same LUT in global memory (t.glut), or a
+// binary search over the ids themselves (t.broker_id[0 .. t.N)). T = any parameter block with those fields.
+template <typename T>
+__device__ __forceinline__ uint32_t ka_id_index(int id, const uint16_t* lut, const T& t) {
+    if (t.lut_mode == KA_LUT_SMEM) {
+        uint32_t off = (uint32_t)id - (uint32_t)t.min_id;
+        return off < t.range ? (uint32_t)lut[off] : KA_DEAD;
+    } else if (t.lut_mode == KA_LUT_GLOBAL) {
+        uint32_t off = (uint32_t)id - (uint32_t)t.min_id;
+        return off < t.range ? (uint32_t)__ldg(&t.glut[off]) : KA_DEAD;
+    } else {
+        int lo = 0, hi = t.N - 1;
+        while (lo <= hi) {
+            int mid = (lo + hi) >> 1;
+            int v = __ldg(&t.broker_id[mid]);
+            if (v == id) return (uint32_t)mid;
+            if (v < id) lo = mid + 1; else hi = mid - 1;
+        }
+        return KA_DEAD;
+    }
+}
+
 __device__ __forceinline__ uint32_t ka_lanemask_lt() {
     uint32_t m;
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));

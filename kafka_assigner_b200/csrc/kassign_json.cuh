@@ -28,6 +28,10 @@ struct KaJsonParams {
     char* json;
     unsigned long long cap;     // bytes of `json`: a fragment that would end beyond it is measured but NOT written
     int first, last;            // write the header before / the trailer after this fragment
+    // changed-rows-only text (IDX kernels): the fragment's rows are sel[0 .. sel_state[1]) (fragment-relative, ascending);
+    // sel_state[0] = rows emitted by earlier fragments, which decides the leading comma
+    const uint32_t* sel;
+    const uint32_t* sel_state;
 };
 
 #define KA_JSON_HEAD "{\"partitions\":["
@@ -54,17 +58,27 @@ __device__ __forceinline__ char* ka_put_str(char* p, const char* s, int n) {
     return p + n;
 }
 
-__device__ __forceinline__ uint32_t ka_json_row_len(const KaJsonParams& p, uint32_t q) {
+// rows this fragment writes, and whether its q-th one is preceded by a comma (it is not the first row of the whole text)
+template <bool IDX> __device__ __forceinline__ uint32_t ka_json_rows(const KaJsonParams& p) { return IDX ? p.sel_state[1] : p.Q; }
+template <bool IDX> __device__ __forceinline__ bool ka_json_comma(const KaJsonParams& p, uint32_t q) {
+    return IDX ? p.sel_state[0] + q > 0 : p.row0 + q > 0;
+}
+
+template <bool IDX>
+__device__ __forceinline__ uint32_t ka_json_row_len(const KaJsonParams& p, uint32_t i) {
+    const uint32_t q = IDX ? p.sel[i] : i;
     const int t = p.topic0 + (int)(q / (uint32_t)p.P), part = (int)(q % (uint32_t)p.P);
     const int len = p.out_len[q];
-    uint32_t n = (p.row0 + q > 0 ? 1u : 0u) + 13u + ka_ndigits(part) + 13u + 11u + (uint32_t)(p.name_off[t + 1] - p.name_off[t]) + 2u;
+    uint32_t n = (ka_json_comma<IDX>(p, i) ? 1u : 0u) + 13u + ka_ndigits(part) + 13u + 11u + (uint32_t)(p.name_off[t + 1] - p.name_off[t]) + 2u;
     for (int i = 0; i < len; ++i) n += ka_ndigits(p.out[(size_t)q * p.S + i]) + (i ? 1u : 0u);
     return n;
 }
-__device__ __forceinline__ void ka_json_row_put(const KaJsonParams& p, uint32_t q, char* w) {
+template <bool IDX>
+__device__ __forceinline__ void ka_json_row_put(const KaJsonParams& p, uint32_t i, char* w) {
+    const uint32_t q = IDX ? p.sel[i] : i;
     const int t = p.topic0 + (int)(q / (uint32_t)p.P), part = (int)(q % (uint32_t)p.P);
     const int len = p.out_len[q];
-    if (p.row0 + q > 0) *w++ = ',';
+    if (ka_json_comma<IDX>(p, i)) *w++ = ',';
     w = ka_put_str(w, "{\"partition\":", 13);
     w = ka_put_int(w, part);
     w = ka_put_str(w, ",\"replicas\":[", 13);
@@ -77,12 +91,15 @@ __device__ __forceinline__ void ka_json_row_put(const KaJsonParams& p, uint32_t 
     ka_put_str(w, "\"}", 2);
 }
 
-// pass 1: text length of every row + per-block sums
+// pass 1: text length of every row + per-block sums. IDX: the grid covers every row of the fragment, the blocks beyond the
+// selected rows (known only on the device) write zero sums.
+template <bool IDX>
 __global__ void __launch_bounds__(256) ka_json_len_kernel(const KaJsonParams p) {
     __shared__ uint32_t wsum[8];
     const uint32_t q = blockIdx.x * 256u + threadIdx.x;
-    uint32_t n = q < p.Q ? ka_json_row_len(p, q) : 0u;
-    if (q < p.Q) p.rowlen[q] = n;
+    const uint32_t nq = ka_json_rows<IDX>(p);
+    uint32_t n = q < nq ? ka_json_row_len<IDX>(p, q) : 0u;
+    if (q < nq) p.rowlen[q] = n;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(KA_FULL, n, o);
     if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = n;
@@ -141,13 +158,15 @@ __global__ void __launch_bounds__(1024) ka_json_scan_kernel(const KaJsonParams p
 // same 16-byte phase as their destination) and copied out with coalesced 16-byte stores; blocks whose text does not fit
 // (very long topic names) write straight to global memory.
 #define KA_JSON_SMEM_BYTES (64 * 1024)
+template <bool IDX>
 __global__ void __launch_bounds__(256) ka_json_write_kernel(const KaJsonParams p) {
     extern __shared__ __align__(16) unsigned char ka_jsmem[];
     __shared__ uint32_t wsum[8];
     if (p.frag[0] + p.frag[1] > p.cap) return;   // caller's buffer too small (uniform: the host reports KA_ERR_LIMIT)
     const uint32_t q = blockIdx.x * 256u + threadIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint32_t n = q < p.Q ? p.rowlen[q] : 0u;
+    const uint32_t nq = ka_json_rows<IDX>(p);
+    const uint32_t n = q < nq ? p.rowlen[q] : 0u;
     uint32_t x = n;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -164,7 +183,7 @@ __global__ void __launch_bounds__(256) ka_json_write_kernel(const KaJsonParams p
     const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(dst) & 15u);
     if (mis + bt <= KA_JSON_SMEM_BYTES) {
         char* stage = reinterpret_cast<char*>(ka_jsmem) + mis;
-        if (q < p.Q) ka_json_row_put(p, q, stage + loc);
+        if (q < nq) ka_json_row_put<IDX>(p, q, stage + loc);
         __syncthreads();
         const uint32_t head = min(bt, (16u - mis) & 15u);       // bytes up to the first 16-byte boundary of dst
         for (uint32_t i = threadIdx.x; i < head; i += 256) dst[i] = stage[i];
@@ -173,8 +192,8 @@ __global__ void __launch_bounds__(256) ka_json_write_kernel(const KaJsonParams p
         uint4* d4 = reinterpret_cast<uint4*>(dst + head);
         for (uint32_t i = threadIdx.x; i < body; i += 256) d4[i] = s4[i];
         for (uint32_t i = head + (body << 4) + threadIdx.x; i < bt; i += 256) dst[i] = stage[i];
-    } else if (q < p.Q) {
-        ka_json_row_put(p, q, dst + loc);
+    } else if (q < nq) {
+        ka_json_row_put<IDX>(p, q, dst + loc);
     }
     if (q == 0 && p.first) ka_put_str(frag, KA_JSON_HEAD, KA_JSON_HEAD_LEN);
     if (q == 0 && p.last) ka_put_str(frag + p.frag[1] - KA_JSON_TAIL_LEN, KA_JSON_TAIL, KA_JSON_TAIL_LEN);

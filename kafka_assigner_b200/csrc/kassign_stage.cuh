@@ -53,22 +53,7 @@ struct KaTab {               // CTA-shared views into the staged broker table
 };
 
 __device__ __forceinline__ uint32_t ka_lookup(int id, const KaTab& tab, const KaSolveParams& p) {
-    if (p.lut_mode == KA_LUT_SMEM) {
-        uint32_t off = (uint32_t)id - (uint32_t)p.min_id;
-        return off < p.range ? (uint32_t)tab.lut[off] : KA_DEAD;
-    } else if (p.lut_mode == KA_LUT_GLOBAL) {
-        uint32_t off = (uint32_t)id - (uint32_t)p.min_id;
-        return off < p.range ? (uint32_t)__ldg(&p.glut[off]) : KA_DEAD;
-    } else {
-        int lo = 0, hi = p.N - 1;
-        while (lo <= hi) {
-            int mid = (lo + hi) >> 1;
-            int v = __ldg(&p.broker_id[mid]);
-            if (v == id) return (uint32_t)mid;
-            if (v < id) lo = mid + 1; else hi = mid - 1;
-        }
-        return KA_DEAD;
-    }
+    return ka_id_index(id, tab.lut, p);
 }
 
 // Per-warp scratch of the conflict-level pass (LEVELS only).
